@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- scans/sec of the FAST-LIO2 iEKF measurement update (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one whole update of one synthetic scan: every iEKF pass of
 update_iterated_dyn_share_modified, kNN included -- ONE launch of the persistent kernel k_update.  Workload at any N: BASELINE.json
@@ -21,6 +21,11 @@ configs[1] ("velodyne.yaml synthetic: 30k pts/scan vs 1M-pt map, 4 iEKF iters").
           restated h_share_model / esekf update) on this box's host cores, bounded sample.
 
 --impl reference times that CPU path as the arm itself (rank 0 only under torchrun).
+
+--dump-outputs DIR writes what the timed path returned for its last step as DIR/<name>.npy (float64 / float32):
+x (26) and P (23x23), the updated state and covariance, and with one process the per-point outputs of the last
+search pass: nearest (Q x 5 x 4, the plane points), nearest_count (Q) and selected (Q, point_selected_surf).  The
+workloads are generated from fixed seeds, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -146,7 +151,7 @@ def cpu_update_loop(pr, n_scans: int, nthreads: int, warm: int = 3):
     The reference's OpenMP loop (laserMapping.cpp:646-650) does not scale to every core count (allocation inside
     KD_TREE::Nearest_Search), so the thread count is calibrated ONCE per process -- 5 scans each at nproc, nproc/2, ...
     >= 4, the candidate with the best median wins -- with the OpenMP threads pinned (OMP_PROC_BIND / OMP_PLACES are set
-    by main() before any OpenMP runtime starts).  Then `warm` untimed scans and n_scans (>= 20) timed ones; the figure
+    by main() before any OpenMP runtime starts).  Then `warm` untimed scans and n_scans timed ones; the figure
     reported is the MEDIAN.  The reference's own default of 3 threads (CMakeLists.txt:23-26: MP_PROC_NUM = 3 on hosts
     with more than 4 cores) is timed beside it.  Returns a dict."""
     from oracle import bind
@@ -172,7 +177,6 @@ def cpu_update_loop(pr, n_scans: int, nthreads: int, warm: int = 3):
         med = {c: float(np.median([one(c) for _ in range(5)])) for c in cands}
         _CPU_CAL[key] = (min(cands, key=lambda c: med[c]), med)
     best, med = _CPU_CAL[key]
-    n_scans = max(20, n_scans)
     for _ in range(max(3, warm)):
         one(best)
     times = [one(best) for _ in range(n_scans)]
@@ -181,7 +185,17 @@ def cpu_update_loop(pr, n_scans: int, nthreads: int, warm: int = 3):
     tree.close()
     return {"times": times, "median_s": float(np.median(times)), "mean_s": float(np.mean(times)), "kind": kind, "threads": best,
             "calibration_ms": {str(c): round(1e3 * v, 2) for c, v in med.items()},
-            "median_s_3_threads": float(np.median(t3)), "x": result.x, "P": result.P}
+            "median_s_3_threads": float(np.median(t3)), "x": result.x, "P": result.P, "result": result}
+
+
+def dump_outputs(out_dir, arrays):
+    """One .npy per array; integer outputs are stored as float32 (exact for counts and flags)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def rot_angle(qa, qb):
@@ -224,6 +238,10 @@ def run_reference(args, rank: int):
                          "note_3_threads": "the reference's compiled-in default MP_PROC_NUM = 3 (CMakeLists.txt:23-26)"},
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        r = c["result"]
+        dump_outputs(args.dump_outputs, {"x": r.x, "P": r.P, "nearest": r.nearest, "nearest_count": r.nearest_cnt,
+                                         "selected": r.selected})
     print(json.dumps(line), flush=True)
     return 0
 
@@ -291,6 +309,11 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     t_wall = time.perf_counter() - t_wall0
     launches = filt.gpu_launches() * args.steps
     x_res, P_res, n_pass = filt.download_state()
+    if args.dump_outputs:
+        outputs = {"x": x_res, "P": P_res}
+        if world == 1:
+            outputs["nearest"], outputs["nearest_count"] = filt.nearest(Q)
+            outputs["selected"] = filt.selected(Q)
     ms_warm = filt.time_resident(args.steps, flush_l2=False)
     # ---- dominant kernel alone
     ms_search = filt.time_search_pass(max(5, args.steps), flush_l2=True) / max(5, args.steps)
@@ -339,7 +362,7 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         if world == 1 and not args.no_cpu_baseline:
             cores = os.cpu_count() or 1
             with c_stdout_to_stderr():
-                c = cpu_update_loop(pr, args.cpu_scans, cores)
+                c = cpu_update_loop(pr, max(20, args.cpu_scans), cores)
             cpu = {"value": 1.0 / c["median_s"], "unit": UNIT, "cores": c["threads"], "kind": c["kind"],
                    "sample": f"median of {len(c['times'])} full scan updates of the same workload ({1e3 * c['median_s']:.2f} ms/scan, mean {1e3 * c['mean_s']:.2f}), "
                              f"threads pinned, thread count calibrated once ({c['calibration_ms']} ms)",
@@ -368,6 +391,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
             "extra": {"value_l2_warm": args.steps / (ms_warm * 1e-3), "wall_s_timed_region": t_wall,
                       "pos_err_vs_truth_m": float(np.abs(x_res[:3] - pr.x_true[:3]).max())},
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
         if parity is not None and not (parity["ok"] and parity["e2e_path"]):
             print("bench.py: the GPU state differs from the CPU reference path beyond 1e-4 -- this number is not valid", file=sys.stderr)
@@ -390,6 +415,7 @@ def main():
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"])
     ap.add_argument("--cpu-scans", type=int, default=20)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     # Pin the OpenMP threads of the CPU reference path (must be in the environment before any OpenMP runtime starts) -- ONLY in a

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -47,10 +48,10 @@ def test_committed_bench_lines_follow_the_contract(path):
         assert d["metric"].split(" (")[0] in want or want.split(" (")[0] in d["metric"]
 
 
-def test_reference_arm_prints_one_contract_line():
+def test_reference_arm_prints_one_contract_line(tmp_path):
     env = dict(os.environ, OMP_NUM_THREADS="4")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
-                          "--workload", "tiny"], capture_output=True, text=True, env=env, timeout=600)
+                          "--workload", "tiny", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1                                  # the ikd-Tree's own printf chatter must not reach stdout
@@ -58,3 +59,8 @@ def test_reference_arm_prints_one_contract_line():
     assert d["impl"] == "reference" and BASE_KEYS <= set(d)
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0
+    assert d["steps"] == 2
+    dumped = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert set(dumped) == {"x", "P", "nearest", "nearest_count", "selected"}
+    assert all(a.dtype in (np.float32, np.float64) for a in dumped.values())
+    assert dumped["x"].shape == (26,) and dumped["P"].shape == (23, 23) and dumped["nearest"].shape == (400, 5, 4)

@@ -5,6 +5,7 @@ import pytest
 
 from fast_lio_b200 import api, synth
 from oracle import bind
+from reference_tape import ReferenceTree
 
 pytestmark = pytest.mark.gpu
 
@@ -126,7 +127,7 @@ def test_localmap_segment_deletes_from_the_map(problems):
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
     ours = api.LocalMap(40.0, 8.0)
     ref = bind.LocalMap(40.0, 8.0)
-    rt = bind.KdTree(pr.map_pts, "auto") if bind.have_ref() else None
+    rt = ReferenceTree("localmap_segment", pr.map_pts)
     pos = np.array(pr.x_true[:3], dtype=np.float64)
     total = 0
     for k in range(12):
@@ -134,7 +135,7 @@ def test_localmap_segment_deletes_from_the_map(problems):
         boxes, n_deleted = ours.segment(pos, g)
         b_ref = ref.segment(pos)
         assert np.array_equal(boxes, b_ref)
-        if rt is not None and len(b_ref):
+        if len(b_ref):
             assert n_deleted == rt.delete_boxes(b_ref)
             assert g.validnum() == rt.validnum()
         total += n_deleted

@@ -1,9 +1,9 @@
-"""kNN parity: the device map against the reference's own ikd-Tree (oracle/_ref) and the port."""
+"""kNN parity: the device map against the reference's own ikd-Tree (its recorded answers, tests/reference_tape.py)."""
 import numpy as np
 import pytest
 
 from fast_lio_b200 import api, synth
-from oracle import bind
+from reference_tape import ReferenceTree
 
 pytestmark = pytest.mark.gpu
 
@@ -24,7 +24,7 @@ def _world_queries(pr):
 def test_knn_matches_reference_ikdtree(problems, name):
     pr = problems(name)
     q = _world_queries(pr)
-    ref = bind.KdTree(pr.map_pts, "auto")
+    ref = ReferenceTree(f"knn_{name}", pr.map_pts)
     rp, rd, rc = ref.knn(q, 5)
     t = api.KdTree(0, 0.5)
     t.Build(pr.map_pts)
@@ -71,7 +71,7 @@ def test_knn_gridded_map_ties():
     q = np.zeros((600, 4), dtype=np.float32)
     q[:, :3] = np.round(rng.uniform(-5, 5, (600, 3)) * 8) / 8          # multiples of 0.125: plenty of equidistant neighbours
     q[:300, 0] += rng.uniform(-0.05, 0.05, 300).astype(np.float32)
-    ref = bind.KdTree(pts, "reference" if bind.have_ref() else "port")
+    ref = ReferenceTree("knn_gridded_map", pts)
     rp, rd, rc = ref.knn(q, 5)
     t = api.KdTree(0, 0.5); t.Build(pts)
     gp, gd, gc = t.Nearest_Search(q, 5)
@@ -99,7 +99,7 @@ def test_knn_planted_ties_are_ordered_by_x():
     pts = np.zeros((len(ps), 4), dtype=np.float32); pts[:, :3] = np.array(ps, dtype=np.float32); pts[:, 3] = np.arange(len(ps))
     pts = pts[rng.permutation(len(pts))]
     q = np.zeros((len(qs), 4), dtype=np.float32); q[:, :3] = np.array(qs, dtype=np.float32)
-    ref = bind.KdTree(pts, "reference" if bind.have_ref() else "port")
+    ref = ReferenceTree("knn_planted_ties", pts)
     rp, rd, rc = ref.knn(q, 5)
     decided, inner_tie = _decided_rows(q, pts, rp, rd)
     assert inner_tie.sum() >= 100                                       # the x rule is exercised

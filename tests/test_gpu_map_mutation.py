@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 from fast_lio_b200 import api, synth
-from oracle import bind
+from reference_tape import ReferenceTree
 from semantics import VoxelMapModel, sort_rows
 
 pytestmark = pytest.mark.gpu
@@ -30,18 +30,12 @@ def check_same_map(g: api.KdTree, r, queries):
     assert np.array_equal(gd, rd)
 
 
-def ref_or_model(pts):
-    if bind.have_ref():
-        return bind.KdTree(pts, "reference", downsample=0.5)
-    pytest.skip("oracle/_ref not available")
-
-
 @pytest.mark.parametrize("name", ["tiny", "small"])
 def test_delete_boxes(problems, name):
     pr = problems(name)
     rng = np.random.default_rng(11)
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
-    r = ref_or_model(pr.map_pts)
+    r = ReferenceTree(f"delete_boxes_{name}", pr.map_pts)
     q = make_batch(rng, pr.map_pts, 256)
     lo = pr.map_pts[:, :3].min(0); hi = pr.map_pts[:, :3].max(0)
     for rep in range(3):
@@ -68,7 +62,7 @@ def test_add_points_downsample(problems, name):
     pr = problems(name)
     rng = np.random.default_rng(7)
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
-    r = ref_or_model(pr.map_pts)
+    r = ReferenceTree(f"add_points_downsample_{name}", pr.map_pts)
     q = make_batch(rng, pr.map_pts, 256)
     for rep in range(4):
         batch = make_batch(rng, pr.map_pts, 1500)
@@ -80,7 +74,7 @@ def test_add_points_no_downsample(problems):
     pr = problems("tiny")
     rng = np.random.default_rng(9)
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
-    r = ref_or_model(pr.map_pts)
+    r = ReferenceTree("add_points_no_downsample", pr.map_pts)
     q = make_batch(rng, pr.map_pts, 128)
     batch = make_batch(rng, pr.map_pts, 2000)
     assert g.Add_Points(batch, False) == r.add(batch, False) == 0
@@ -96,10 +90,9 @@ def test_add_into_non_downsampled_map_and_model():
     m = VoxelMapModel(pts, 0.5)
     assert g.Add_Points(batch, True) == m.add_points(batch, True)
     assert np.array_equal(sort_rows(g.flatten()), sort_rows(m.flatten()))
-    if bind.have_ref():
-        r = bind.KdTree(pts, "reference", downsample=0.5)
-        r.add(batch, True)
-        assert np.array_equal(sort_rows(g.flatten()), sort_rows(r.flatten()))
+    r = ReferenceTree("add_into_non_downsampled_map", pts)
+    r.add(batch, True)
+    assert np.array_equal(sort_rows(g.flatten()), sort_rows(r.flatten()))
 
 
 def test_overflow_chain_and_rebuild():
@@ -129,7 +122,7 @@ def test_stream_of_scans_matches_reference(problems):
     pr = problems("small")
     rng = np.random.default_rng(33)
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
-    r = ref_or_model(pr.map_pts)
+    r = ReferenceTree("stream_of_scans_map", pr.map_pts)
     for step in range(5):
         batch = make_batch(rng, pr.map_pts, 800)
         assert g.Add_Points(batch[:600], True) == r.add(batch[:600], True)
@@ -172,14 +165,14 @@ def test_acquire_removed_points_and_add_point_boxes(problems):
     q = np.ascontiguousarray(np.array(added_back[:50], dtype=np.float32))
     gp, gd, gc = g.Nearest_Search(q, 1)
     assert (gd[:, 0] == 0).all()
-    if bind.have_ref():                                         # without intervening inserts the reference restores the map exactly
-        g2 = api.KdTree(0, 0.5); g2.Build(pr.map_pts)
-        g2.Delete_Point_Boxes(boxes)
-        assert g2.Add_Point_Boxes(boxes) == n_del
-        assert np.array_equal(sort_rows(g2.flatten()), before)
-        qq = make_batch(rng, pr.map_pts, 200)
-        r = bind.KdTree(pr.map_pts, "reference", downsample=0.5)
-        assert np.array_equal(g2.Nearest_Search(qq, 5)[1], r.knn(qq, 5)[1])
+    # without intervening inserts the reference restores the map exactly
+    g2 = api.KdTree(0, 0.5); g2.Build(pr.map_pts)
+    g2.Delete_Point_Boxes(boxes)
+    assert g2.Add_Point_Boxes(boxes) == n_del
+    assert np.array_equal(sort_rows(g2.flatten()), before)
+    qq = make_batch(rng, pr.map_pts, 200)
+    r = ReferenceTree("add_point_boxes", pr.map_pts)
+    assert np.array_equal(g2.Nearest_Search(qq, 5)[1], r.knn(qq, 5)[1])
 
 
 def test_directory_lists_grow_and_slots_are_reused():

@@ -4,15 +4,13 @@ import numpy as np
 import pytest
 
 from fast_lio_b200 import api, synth
-from oracle import bind
+from reference_tape import ReferenceTree
 from semantics import map_incremental, sort_rows
 
 pytestmark = pytest.mark.gpu
 
 
 def test_map_incremental_matches_reference(problems):
-    if not bind.have_ref():
-        pytest.skip("oracle/_ref not available")
     pr = problems("small")
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
     f = api.Esekf(g, max_points=len(pr.scan), max_iter=pr.cfg.max_iter)
@@ -20,7 +18,7 @@ def test_map_incremental_matches_reference(problems):
     near, cnt = f.nearest(len(pr.scan))
     n_add, n_no, added = f.map_incremental(0.5, True)
     # CPU reference pipeline from the same update result
-    r = bind.KdTree(pr.map_pts, "reference", downsample=0.5)
+    r = ReferenceTree("map_incremental_small", pr.map_pts, downsample=0.5)      # fed the device's points: new bits need a new tape
     to_add, no_need = map_incremental(pr.scan, x, near, cnt, 0.5, True)
     assert (n_add, n_no) == (len(to_add), len(no_need))
     assert added == r.add(to_add, True)
@@ -31,13 +29,11 @@ def test_map_incremental_matches_reference(problems):
 
 def test_stream_of_scans(problems):
     """5 scans: the sensor advances 0.1 m per scan; state and map of the device pipeline track the CPU pipeline."""
-    if not bind.have_ref():
-        pytest.skip("oracle/_ref not available")
     pr = problems("small")
     scene = pr.scene
     g = api.KdTree(0, 0.5); g.Build(pr.map_pts)
     f = api.Esekf(g, max_points=2000, max_iter=3)
-    r = bind.KdTree(pr.map_pts, "reference", downsample=0.5)
+    r = ReferenceTree("stream_of_scans_small", pr.map_pts, downsample=0.5)
     x_g = pr.x_prior.copy(); x_c = pr.x_prior.copy()
     P_g = pr.P_prior.copy(); P_c = pr.P_prior.copy()
     for step in range(5):
@@ -49,7 +45,7 @@ def test_stream_of_scans(problems):
         # crude prediction: carry the state over, inflate the covariance
         P_g = P_g + np.eye(23) * 1e-4; P_c = P_c + np.eye(23) * 1e-4
         x_g, P_g, _ = f.update_iterated_dyn_share_modified(scan, x_g, P_g, pr.R)
-        o = bind.update_iterated(r, scan, x_c, P_c, 3, pr.R, pr.limit, 0)
+        o = r.update_iterated(scan, x_c, P_c, 3, pr.R, pr.limit, 0)
         x_c, P_c = o.x, o.P
         assert np.abs(x_g[:3] - x_c[:3]).max() <= 1e-4 and np.abs(x_g[3:7] - x_c[3:7]).max() <= 1e-4
         n_add, n_no, added = f.map_incremental(0.5, True)

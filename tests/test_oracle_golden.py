@@ -8,6 +8,7 @@ import pytest
 
 from fast_lio_b200 import synth
 from oracle import bind
+from reference_tape import ReferenceTree
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -33,11 +34,9 @@ def test_generator_is_stable(problems, name):
 @pytest.mark.parametrize("name", ["tiny", "small"])
 @pytest.mark.parametrize("backend", ["port", "reference"])
 def test_knn_golden(problems, name, backend):
-    if backend == "reference" and not bind.have_ref():
-        pytest.skip("oracle/_ref not built")
     g = np.load(os.path.join(GOLD, f"{name}.npz"))
     pr = problems(name)
-    t = bind.KdTree(pr.map_pts, backend)
+    t = ReferenceTree(f"knn_{name}", pr.map_pts) if backend == "reference" else bind.KdTree(pr.map_pts, backend)
     p, d, c = t.knn(world_queries(pr), 5)
     assert np.array_equal(c, g["knn_cnt"]) and np.array_equal(d, g["knn_d2"]) and np.array_equal(p, g["knn_pts"])
 

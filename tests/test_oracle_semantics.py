@@ -1,20 +1,18 @@
-"""CPU: pin the oracle pieces against each other and against the reference's own ikd-Tree."""
+"""CPU: pin the oracle pieces against each other and against the reference's own ikd-Tree (its recorded answers)."""
 import numpy as np
 import pytest
 
 from fast_lio_b200 import synth
 from oracle import bind
+from reference_tape import ReferenceTree
 from semantics import VoxelMapModel, sort_rows
 
-needs_ref = pytest.mark.skipif(not bind.have_ref(), reason="oracle/_ref (reference ikd-Tree) not built")
 
-
-@needs_ref
 def test_port_knn_equals_reference_ikdtree(problems):
     pr = problems("small")
     q = pr.map_pts[::7].copy()
     q[:, :3] += 0.21
-    a = bind.KdTree(pr.map_pts, "reference")
+    a = ReferenceTree("port_knn_small", pr.map_pts)
     b = bind.KdTree(pr.map_pts, "port")
     pa, da, ca = a.knn(q)
     pb, db, cb = b.knn(q)
@@ -32,11 +30,10 @@ def test_knn_port_brute_force():
         assert np.array_equal(d[i], np.sort(dd)[:5])
 
 
-@needs_ref
 def test_mutation_model_equals_reference_ikdtree():
     rng = np.random.default_rng(4)
     pts = rng.uniform(-4, 4, (2500, 4)).astype(np.float32)
-    r = bind.KdTree(pts, "reference", downsample=0.5)
+    r = ReferenceTree("mutation_model", pts, downsample=0.5)
     m = VoxelMapModel(pts, 0.5)
     for rep in range(3):
         batch = rng.uniform(-5, 5, (700, 4)).astype(np.float32)
